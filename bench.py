@@ -14,6 +14,9 @@ insert/increment) over the whole synthetic input, into a zeroed table.
   cpu_baseline  the reference binary (oracle/_ref/jellyfish, all host threads) on a bounded
                 sample of the same workload
 
+--dump-outputs DIR writes what the last timed step computed (see dump_outputs) as DIR/<name>.npy; the
+inputs are generated from fixed seeds, so two builds given the same arguments can be compared file by file.
+
 Workload (N=1, default --config k21): BASELINE configs[1], k=21 canonical, 10 Gbp synthetic FASTA.
 configs[1] names a "4 G-entry hash", which cannot hold the ~9.98e9 distinct 21-mers of 10 Gbp iid
 sequence: the reference doubles it twice to 2^34 slots.  The bench therefore sizes the table at
@@ -248,6 +251,7 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--dump", action="store_true", help="also time one full sorted dump (Writing phase) to /dev/null-like sink")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write what the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
     cfg = CONFIGS[args.config]
     args.k = args.k or cfg["k"]
@@ -340,6 +344,8 @@ def main():
     xtrace = counter.records.trace if counter is not None and counter.records is not None else None     # (stages of the last step)
     clocks = sampler.stop()
     launches = lib.jfgpu_kernel_launches() - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, hc, st, text, n_bases, k, rank if world > 1 else None)
     tot = torch.tensor([st["kmers"], st["inserted"], st["distinct"]], dtype=torch.int64, device=dev)
     if world > 1:
         dist.all_reduce(tot)          # keys are inserted by their owner: only the sums must agree
@@ -490,6 +496,36 @@ def main():
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+OUTPUT_SAMPLE = 1 << 16          # k-mers of the input whose counts --dump-outputs writes
+OUTPUT_SEED = 0x5EED0F0B
+
+
+def dump_outputs(out_dir, hc, st, text, n_bases, k, rank):
+    """What a caller of the timed path receives from its last step, as float64 arrays (every value is an integer below 2^53):
+      stats             kmers, inserted, distinct of the statistics done() returns
+      histogram         distinct k-mers by count, counts of 1023 and more in the last bin (`jellyfish histo`)
+      sample_positions  OUTPUT_SAMPLE positions in the sequence, drawn with OUTPUT_SEED
+      sample_counts     the table's count of the k-mer starting at each of them
+    Written as DIR/<name>.npy, DIR/<name>_rank<r>.npy for the shard of rank r of a sharded run (keys of other shards count 0)."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    # the text is one record, 70-column lines: base q sits at offset (header line) + q + q // 70
+    head = text[:4096].cpu().numpy().tobytes()
+    first = head.index(b"\n") + 1
+    pos = np.sort(np.random.default_rng(OUTPUT_SEED).integers(0, n_bases - k + 1, size=OUTPUT_SAMPLE))
+    q = pos[:, None] + np.arange(k)
+    idx = torch.from_numpy((first + q + q // 70).reshape(-1)).to(text.device)
+    bases = text[idx].cpu().numpy().reshape(OUTPUT_SAMPLE, k)
+    assert np.isin(bases, np.frombuffer(b"ACGT", dtype=np.uint8)).all(), "sampled k-mers are not all ACGT: text layout changed"
+    counts = hc.get_many([row.tobytes().decode() for row in bases])
+    suffix = "" if rank is None else "_rank%d" % rank
+    arrays = {"stats": [st["kmers"], st["inserted"], st["distinct"]], "histogram": hc.histogram(1024),
+              "sample_positions": pos, "sample_counts": counts}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def sharded_parity_check(world, rank, local_rank):

@@ -1,9 +1,10 @@
 #!/usr/bin/env python
 """Differential fuzz of the C restatement (oracle/_ref/jf_oracle) against the UNMODIFIED reference
 (oracle/_ref/jellyfish): random switches and small random inputs, header keys and record bodies
-compared byte for byte. Build-container tool (needs the reference binary); failures print the
-command line so that the case can be added to tests/cases.py.
-    python scripts/fuzz_oracle.py [N] [SEED]
+compared byte for byte; failures print the command line so that the case can be added to tests/cases.py.
+    python scripts/fuzz_oracle.py [N] [SEED] [--record FILE | --replay FILE]
+Without a switch the reference binary is asked directly.  --record also keeps its answers (exit status, header digest, body
+md5) in FILE; --replay takes them from FILE instead of the binary, so the comparison runs where the reference does not.
 """
 import os
 import random
@@ -15,8 +16,16 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 import jfutil  # noqa: E402
 
-n_iter = int(sys.argv[1]) if len(sys.argv) > 1 else 100
-rng = random.Random(int(sys.argv[2]) if len(sys.argv) > 2 else 1)
+argv = sys.argv[1:]
+mode, golden = "live", None
+for sw in ("--record", "--replay"):
+    if sw in argv:
+        i = argv.index(sw)
+        mode, golden = sw[2:], argv[i + 1]
+        del argv[i:i + 2]
+n_iter = int(argv[0]) if len(argv) > 0 else 100
+rng = random.Random(int(argv[1]) if len(argv) > 1 else 1)
+ref = jfutil.RefLog(golden, mode)
 
 
 def rand_seq(n, alphabet="ACGT"):
@@ -54,8 +63,23 @@ def rand_fastq(path):
     open(path, "w").write("".join(out))
 
 
+def db_answer(rc, path):
+    """What the comparison needs of a count run: success, and the header digest and body of the database."""
+    if rc != 0:
+        return {"ok": False}
+    h, b = jfutil.split_db(path)
+    return {"ok": True, "header": jfutil.semantic_md5(h), "md5": jfutil.md5(b), "len": len(b)}
+
+
+def run_ref(cmd, out):
+    return db_answer(subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.PIPE).returncode, out)
+
+
 bad = 0
 with tempfile.TemporaryDirectory() as d:
+    def rel(args):
+        return " ".join(os.path.relpath(a, d) if a.startswith(d) else a for a in args)
+
     for it in range(n_iter):
         files = []
         kinds = sorted(rng.random() < 0.3 for _ in range(rng.randrange(1, 4)))   # FASTA files first (see -Q note in tests/cases.py)
@@ -90,31 +114,31 @@ with tempfile.TemporaryDirectory() as d:
         elif u < 0.2:
             bc = os.path.join(d, "f.bc")
             bargs = ["-m", str(k), "-s", rng.choice(["100", "5k", "100k"]), "-f", rng.choice(["0.001", "0.05", "0.3"])] + (["-C"] if "-C" in args else [])
-            r1 = subprocess.run([jfutil.REF_JF, "bc", "-t", "2"] + bargs + ["-o", bc] + files[:2], stdout=subprocess.PIPE, stderr=subprocess.PIPE)
+            r1 = ref.answer("bc " + rel(bargs + files[:2]), lambda: run_ref([jfutil.REF_JF, "bc", "-t", "2"] + bargs + ["-o", bc] + files[:2], bc))
             r2 = subprocess.run([jfutil.ORACLE_C, "bc"] + bargs + ["-o", bc + ".o"] + files[:2], stdout=subprocess.PIPE, stderr=subprocess.PIPE)
-            if r1.returncode == 0 and r2.returncode == 0:
-                if jfutil.split_db(bc)[1] != jfutil.split_db(bc + ".o")[1]:
+            if r1["ok"] and r2.returncode == 0:
+                if r1["md5"] != jfutil.md5(jfutil.split_db(bc + ".o")[1]):
                     bad += 1
                     print("MISMATCH #%d: bc files differ: bc %s %s" % (it, " ".join(bargs), " ".join(files[:2])))
+                if mode == "replay":          # the restatement's file stands in for the reference's: the same counters
+                    os.replace(bc + ".o", bc)
                 args += ["--bc", bc]
         r_db, o_db = os.path.join(d, "r.jf"), os.path.join(d, "o.jf")
         for f in (r_db, o_db):
             if os.path.exists(f):
                 os.remove(f)
-        rr = subprocess.run([jfutil.REF_JF, "count", "-t", "1"] + args + ["-o", r_db] + files, stdout=subprocess.PIPE, stderr=subprocess.PIPE)
+        rr = ref.answer("count " + rel(args + files), lambda: run_ref([jfutil.REF_JF, "count", "-t", "1"] + args + ["-o", r_db] + files, r_db))
         ro = subprocess.run([jfutil.ORACLE_C, "count"] + args + ["-o", o_db] + files, stdout=subprocess.PIPE, stderr=subprocess.PIPE)
         ok = True
         why = ""
-        if (rr.returncode == 0) != (ro.returncode == 0):
-            ok, why = False, "exit status ref %d oracle %d: %s | %s" % (rr.returncode, ro.returncode, rr.stderr[-200:], ro.stderr[-200:])
-        elif rr.returncode == 0:
-            h1, b1 = jfutil.split_db(r_db)
+        if rr["ok"] != (ro.returncode == 0):
+            ok, why = False, "exit status: ref %s, oracle %d: %s" % ("ok" if rr["ok"] else "failed", ro.returncode, ro.stderr[-200:])
+        elif rr["ok"]:
             h2, b2 = jfutil.split_db(o_db)
-            if jfutil.semantic(h1) != jfutil.semantic(h2):
-                diff = [kk for kk in jfutil.SEMANTIC_KEYS if h1.get(kk) != h2.get(kk)]
-                ok, why = False, "header keys differ: %s (ref %s oracle %s)" % (diff, [str(h1.get(kk))[:60] for kk in diff], [str(h2.get(kk))[:60] for kk in diff])
-            elif b1 != b2:
-                ok, why = False, "bodies differ (%d vs %d bytes)" % (len(b1), len(b2))
+            if rr["header"] != jfutil.semantic_md5(h2):
+                ok, why = False, "semantic header keys differ"
+            elif rr["md5"] != jfutil.md5(b2):
+                ok, why = False, "bodies differ (%d vs %d bytes)" % (rr["len"], len(b2))
         if not ok:
             bad += 1
             keep = os.path.join("/tmp", "fuzz_fail_%d" % it)
@@ -124,5 +148,6 @@ with tempfile.TemporaryDirectory() as d:
                 subprocess.run(["cp", f, keep])
                 kept.append(os.path.join(keep, os.path.basename(f)))
             print("MISMATCH #%d: %s\n   count %s %s" % (it, why, " ".join(args), " ".join(kept)))
+ref.close()
 print("%d iterations, %d mismatches" % (n_iter, bad))
 sys.exit(1 if bad else 0)

@@ -156,3 +156,20 @@ DISK_CASES = {
     "disk_k21_LU": (["-m", "21", "-s", "100k", "--disk", "-C", "-L", "2"], ["plain.fa", "multi.fa", "plain.fa"]),
     "disk_k17_c3": (["-m", "17", "-s", "30k", "--disk", "-c", "3", "--out-counter-len", "2"], ["multi.fa", "multi2.fa"]),
 }
+
+# The host-side readers (dump, histo, stats) against the reference's on one database (test_host.py), and the merges
+# (merge_main.cc:31-37, merge_files.cc:45-176) of test_host.py::test_merge_matches_reference: name -> count switches and inputs
+# of the merged databases; (tag, merge switches, databases) of every merge; the --disk run whose intermediate files the
+# reference wrote (tests/golden/disk_parts/).  The reference's answers: tests/golden/golden_tools.json.
+READER_COMMANDS = (["dump", "-c"], ["dump"], ["dump", "-c", "-t", "-L", "2", "-U", "50"], ["histo"], ["histo", "-l", "2", "-h", "20", "-i", "3", "-f"],
+                   ["stats"], ["stats", "-L", "2"])
+MERGE_COUNTS = (("a", ["-m", "17", "-s", "1M", "-C"], ["multi.fa"]),
+                ("b", ["-m", "17", "-s", "1M", "-C"], ["multi2.fa"]),
+                ("c", ["-m", "17", "-s", "1M", "-C"], ["multi.fa", "dangling.fa"]),
+                ("ta", ["-m", "17", "-s", "1M", "-C", "--text"], ["multi.fa"]),
+                ("tb", ["-m", "17", "-s", "1M", "-C", "--text"], ["multi2.fa", "dangling.fa"]))
+MERGE_OPS = (("sum", [], ["a", "b"]), ("min", ["--min"], ["a", "c"]), ("min0", ["-m", "-L", "0"], ["a", "b"]), ("max", ["--max"], ["a", "b", "c"]),
+             ("maxLU", ["-M", "-L", "2", "-U", "3"], ["a", "c"]), ("sum3", ["-L", "2"], ["a", "b", "c"]), ("min3", ["-m"], ["c", "a", "c"]),
+             ("jaccard_ac", ["--jaccard"], ["a", "c"]), ("jaccard_ab", ["--jaccard"], ["a", "b"]), ("jaccard_abc", ["--jaccard"], ["a", "b", "c"]),
+             ("tsum", [], ["ta", "tb"]), ("tmin", ["-m"], ["ta", "tb"]), ("tmaxL", ["-M", "-L", "2"], ["ta", "tb"]))
+DISK_PARTS_COUNT = (["-m", "21", "-s", "1k", "-C", "--disk", "--no-merge", "-t", "2"], "dangling.fa")

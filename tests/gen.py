@@ -22,6 +22,36 @@ def fasta(seq, line=70, name=b"read1", eol=b"\n"):
     return b"".join(out)
 
 
+def generate_sequence(prefix, seed, *lengths):
+    """The FASTA files of the reference's `generate_sequence -o PREFIX -s SEED LEN...`, byte for byte: one MT19937 stream
+    (seeded as init_genrand, its first 37 words skipped), 16 bases per 32-bit word from the low bits up (A, C, G, T), one
+    record '>read1' in 70-column lines followed by an empty record '>read2'.  Several lengths -> PREFIX_0.fa, PREFIX_1.fa, ...
+    from the same stream, each file starting on a fresh word.  -> list of paths."""
+    import numpy as np
+    rs = np.random.RandomState(seed & 0xFFFFFFFF)
+    rs.randint(0, 1 << 32, size=37, dtype=np.uint64)
+    lut = np.frombuffer(b"ACGT", dtype=np.uint8)
+    paths = []
+    for i, n in enumerate(lengths):
+        path = "%s_%d.fa" % (prefix, i) if len(lengths) > 1 else prefix + ".fa"
+        words = rs.randint(0, 1 << 32, size=(n + 15) // 16, dtype=np.uint64).astype(np.uint32)
+        shifts = np.arange(0, 32, 2, dtype=np.uint32)
+        seq = lut[((words[:, None] >> shifts) & 3).reshape(-1)[:n]]
+        full = n // 70
+        with open(path, "wb") as f:
+            f.write(b">read1\n")
+            body = np.empty((full, 71), dtype=np.uint8)
+            body[:, :70] = seq[:full * 70].reshape(-1, 70)
+            body[:, 70] = 10
+            f.write(body.tobytes())
+            if n > full * 70:
+                f.write(seq[full * 70:].tobytes() + b"\n")
+            if n:
+                f.write(b">read2\n")
+        paths.append(path)
+    return paths
+
+
 def make_all(d):
     """-> dict name -> path.  Sizes are small so that the CPU reference runs in seconds."""
     f = {}

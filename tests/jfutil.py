@@ -55,8 +55,63 @@ def records(header, body):
     return out
 
 
-def generate(prefix, seed, *lengths, extra=()):
-    run([REF_GEN, "-o", prefix, "-s", str(seed)] + list(extra) + [str(x) for x in lengths])
+def generate(prefix, seed, *lengths):
+    """The files of the reference's `generate_sequence -o PREFIX -s SEED LEN...` (restated in tests/gen.py)."""
+    import gen
+    return gen.generate_sequence(prefix, seed, *lengths)
+
+
+def golden(name):
+    with open(os.path.join(ROOT, "tests", "golden", name)) as f:
+        return json.load(f)
+
+
+def db_digest(path):
+    """What a comparison of two databases looks at: the semantic header keys and the record body."""
+    h, b = split_db(path)
+    return {"header": semantic(h), "body_md5": md5(b), "body_len": len(b)}
+
+
+def semantic_md5(header):
+    """Digest of the semantic header keys (stored in place of the keys where a golden file holds many headers)."""
+    return md5(json.dumps(semantic(header), sort_keys=True).encode())
+
+
+def records_md5(recs):
+    """Digest of a set of (key, count) records, independent of their order in the file."""
+    return md5(json.dumps(sorted(recs)).encode())
+
+
+class RefLog(object):
+    """The answers of the reference binary, in the order they were asked for.  live: ask the binary; record: ask it and keep
+    the answers in `path`; replay: read them back from `path` (a golden file), so that a comparison with the reference runs
+    where the reference does not.  `what` names the question (paths relative to the run's directory); a replayed answer to
+    another question means the golden file no longer matches the cases and raises."""
+
+    def __init__(self, path=None, mode="live"):
+        assert mode in ("live", "record", "replay")
+        self.path, self.mode, self.i = path, mode, 0
+        self.items = json.load(open(path)) if mode == "replay" else []
+
+    def answer(self, what, ask):
+        if self.mode != "replay":
+            v = ask()
+            if self.mode == "record":
+                self.items.append([what, v])
+            return v
+        if self.i >= len(self.items) or self.items[self.i][0] != what:
+            raise RuntimeError("%s out of step at answer %d: golden %r, asked %r" % (
+                self.path, self.i, self.items[self.i][0] if self.i < len(self.items) else None, what))
+        self.i += 1
+        return self.items[self.i - 1][1]
+
+    def close(self):
+        if self.mode == "record":
+            with open(self.path, "w") as f:
+                json.dump(self.items, f, separators=(",", ":"))
+                f.write("\n")
+        elif self.mode == "replay" and self.i != len(self.items):
+            raise RuntimeError("%s: %d answers recorded, %d asked for" % (self.path, len(self.items), self.i))
 
 
 def subst(args, files):
